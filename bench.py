@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the E4S synthesis hot path (BASELINE.json configs[1]: 1024x1024 synthesis, batch 16 per GPU).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one mask-guided synthesis pass (`Net3.gen_img`, the call scripts/face_swap.py:273 and
@@ -14,6 +14,11 @@ pinned HOST buffers (codes + uint8 label maps copied H2D, final images copied D2
 `roofline` = the modulated-convolution kernels' achieved TFLOP/s (algorithmic FLOPs / CUDA-event time inside
 the timed region) against the measured bf16 tensor peak; `cpu_baseline` = one full 1024x1024 face through the
 reference-structured CPU oracle on the host cores.  `--impl reference` times that CPU path alone.
+
+`--dump-outputs DIR` writes what the timed path returned in its last timed step (the images; with N ranks, rank 0's, which
+are all N ranks' images when `--gather` is set) to DIR/image.npy.  Weights,
+codes, masks and the noise of the timed steps are seeded, so runs with the same arguments get the same inputs and the dumps
+of two builds can be compared element for element.
 """
 from __future__ import annotations
 
@@ -92,7 +97,13 @@ def parse_args():
     ap.add_argument("--inversion-steps", type=int, default=20,
                     help="also time this many steps of the texture-vector optimisation (scripts/optimization.py:209-232, "
                          "l2 loss) on one face per GPU; 0 disables")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the images of the last one as DIR/image.npy (float32; a fixed, seeded "
+                         "sample of them when they exceed %d elements; with N ranks, rank 0's images)" % DUMP_MAX_ELEMENTS)
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 # ------------------------------------------------------------------------------------------ inputs
@@ -313,8 +324,10 @@ def run_reference(args):
         _, state, _ = cpu_reference_face(args.size, args.ncls, state)
     times = []
     for i in range(args.steps):
-        dt, state, _ = cpu_reference_face(args.size, args.ncls, state, seed=2 + i)
+        dt, state, img = cpu_reference_face(args.size, args.ncls, state, seed=2 + i)
         times.append(dt)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"image": img})
     sec = float(np.mean(times))
     val = 1.0 / sec
     cores = torch.get_num_threads()
@@ -409,10 +422,11 @@ def run_ours(args):
         if profile_range:                             # ncu --profile-from-start off: the launch list is the timed region
             torch.cuda.profiler.start()
         K.LaunchStats.reset(timing=kernel_timing)
+        torch.cuda.manual_seed(700 + rank)            # the timed steps' noise maps do not depend on what ran before them
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(steps):
-            fn()
+            out = fn()
         if finish is not None:
             finish()                                  # the timing stream waits for the copy streams
         e1.record()
@@ -427,15 +441,18 @@ def run_ours(args):
             t = torch.tensor([ms], device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t.item())
-        return ms, clocks, launches, summary
+        return ms, clocks, launches, summary, out
 
-    ms, clocks, launches, _ = timed(step_device, args.steps, args.warmup, sample_clocks=True)
+    ms, clocks, launches, _, last = timed(step_device, args.steps, args.warmup, sample_clocks=True)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"image": last})        # before the next pass overwrites the graph's static image
+    del last
     faces = B * world * args.steps
     value = faces / (ms * 1e-3)
     # the same K steps on eager launches: once clean, once with CUDA events around EVERY launch (per-kernel times for the
     # roofline / `kernels` breakdown; the events cost time themselves, so this pass is not the reported value)
-    ms_eager, _, launches_eager, _ = timed(step_eager, args.steps, args.warmup)
-    ms_inst, _, _, summary = timed(step_eager, args.steps, args.warmup, kernel_timing=True)
+    ms_eager, _, launches_eager, _, _ = timed(step_eager, args.steps, args.warmup)
+    ms_inst, _, _, summary, _ = timed(step_eager, args.steps, args.warmup, kernel_timing=True)
     eager = {"value": faces / (ms_eager * 1e-3), "ms_per_step": ms_eager / args.steps, "gpu_launches": launches_eager,
              "ms_per_step_with_per_launch_events": ms_inst / args.steps}
 
@@ -450,7 +467,7 @@ def run_ours(args):
     leg_done("setup+value+eager passes")
     e2e = None
     if not args.no_e2e:
-        ms2, _, _, _ = timed(step_e2e, args.steps, max(args.warmup, 3), finish=pipe.drain)
+        ms2, _, _, _, _ = timed(step_e2e, args.steps, max(args.warmup, 3), finish=pipe.drain)
         e2e = {"value": faces / (ms2 * 1e-3), "unit": "faces/s", "ms_per_step": ms2 / args.steps,
                "h2d_bytes_per_step": int(codes_host.numel() * 4 + labels_host.numel()),
                "d2h_bytes_per_step": int(images_host.numel() * 4),
@@ -816,6 +833,21 @@ def run_ours(args):
         emit(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_MAX_ELEMENTS = 1 << 23                          # 32 MiB of float32: a dump stays below 64 MB
+
+
+def dump_outputs(outdir: str, arrays) -> None:
+    """Each tensor as <outdir>/<name>.npy in float32.  One with more than DUMP_MAX_ELEMENTS elements is replaced by its
+    elements at a fixed, seeded set of flat indices (sorted, 1-D): the same set for the same shape in every run."""
+    os.makedirs(outdir, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach().float()
+        if t.numel() > DUMP_MAX_ELEMENTS:
+            idx = torch.randint(t.numel(), (DUMP_MAX_ELEMENTS,), generator=torch.Generator().manual_seed(0)).sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        np.save(os.path.join(outdir, name + ".npy"), t.cpu().numpy())
 
 
 _OUT_FD = None

@@ -2,6 +2,7 @@
 import math
 import types
 
+import numpy as np
 import pytest
 import torch
 import torch.nn.functional as F
@@ -72,7 +73,7 @@ def test_local_mlps_need_the_gpu_kernel():
         net.cal_style_codes(torch.randn(1, 12, 1280))
 
 
-def test_bench_reference_arm_emits_contract_line():
+def test_bench_reference_arm_emits_contract_line(tmp_path):
     """`bench.py --impl reference` (the CPU arm the driver runs beside ours) prints one JSON line with the contract's keys;
     run here at 64x64 so that it takes seconds."""
     import json
@@ -81,13 +82,15 @@ def test_bench_reference_arm_emits_contract_line():
     import sys
     from conftest import ROOT
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--size", "64", "--steps", "1",
-                          "--warmup", "1"], capture_output=True, text=True, timeout=600)
+                          "--warmup", "1", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=600)
     assert out.returncode == 0, out.stderr[-2000:]
     line = json.loads(out.stdout.strip().splitlines()[-1])
     assert line["impl"] == "reference" and line["unit"] == "faces/s" and line["higher_is_better"] is True and line["value"] > 0
     assert line["cpu_baseline"]["kind"] == "port" and line["cpu_baseline"]["cores"] >= 1 and line["cpu_baseline"]["value"] == line["value"]
     assert line["e2e"] == {"value": line["value"], "unit": "faces/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
     assert line["steps"] == 1 and line["n_gpus"] == 1 and line["gpu_launches"] == 0
+    img = np.load(tmp_path / "image.npy")
+    assert img.dtype == np.float32 and img.shape == (1, 3, 64, 64) and np.isfinite(img).all()
 
 
 def test_dropin_overlay_resolves_reference_import_paths():

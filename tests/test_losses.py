@@ -14,7 +14,6 @@ from conftest import ROOT, assert_close
 
 DEV = "cuda:0"
 SALT = 11                                             # the salt oracle/make_golden_losses.py used
-SHIPPED_UNET = "/root/reference/pretrained_ckpts/auxiliray/model.pth"      # exists only in the build container
 
 
 @pytest.fixture(scope="module")
@@ -47,35 +46,49 @@ def test_loss_oracle_matches_reference_vectors(gold):
             assert_close(f[:, :4096], gold[f"id/feats{i}"], 2e-5, f"id feats {i}")
 
 
-@pytest.mark.skipif(not os.path.exists(SHIPPED_UNET), reason="the reference's shipped parsing checkpoint is only in the build container")
-def test_shipped_parsing_checkpoint_loads_and_matches(gold):
-    """The one loss network whose weights ship with the reference: strict state-dict load into the product module and the
-    oracle's features / loss against the reference's."""
+def test_shipped_parsing_checkpoint_layout_and_first_stages(gold):
+    """The one loss network whose weights ship with the reference: its checkpoint's key / shape layout (which the seeded
+    stand-in shares) loads strictly into the product module, and with the checkpoint's first two encoder stages
+    (tests/golden/parsing_checkpoint.npz) the oracle's and the product module's features at those depths equal the
+    reference's features with the whole checkpoint."""
     from e4s_b200.criteria import FaceParsingLoss
-    sd = torch.load(SHIPPED_UNET, map_location="cpu")
+    ck = np.load(os.path.join(ROOT, "tests", "golden", "parsing_checkpoint.npz"))
+    shapes = {k[len("shape/"):]: tuple(int(s) for s in ck[k]) for k in ck.files if k.startswith("shape/")}
+    seeded = LO.loss_states(SALT)["parsing"]
+    assert shapes == {k[len("G."):]: tuple(v.shape) for k, v in seeded.items()}
+    sd = {k: torch.from_numpy(ck["value/" + k]) if "value/" + k in ck.files else seeded["G." + k] for k in shapes}
     m = FaceParsingLoss(types.SimpleNamespace())
     m.G.load_state_dict(sd, strict=True)
-    real = {"G." + k: v for k, v in sd.items()}
-    img, recon, far = LO.golden_inputs()
+    img, _, _ = LO.golden_inputs()
     with torch.no_grad():
-        _close(LO.parsing_loss(real, recon, img), gold["parsing_shipped/near"])
-        _close(LO.parsing_loss(real, far, img), gold["parsing_shipped/far"])
-        for i, f in enumerate(LO.parsing_extract_feats(real, img)):
-            assert_close(f[:, :4096], gold[f"parsing_shipped/feats{i}"], 2e-5, f"parsing feats {i}")
-        _close(m(recon, img)[0], gold["parsing_shipped/near"])
+        oracle = LO.parsing_extract_feats({"G." + k: v for k, v in sd.items()}, img)
+        ours = m.extract_feats(img)
+    for i in range(2):
+        assert_close(oracle[i][:, :4096], gold[f"parsing_shipped/feats{i}"], 2e-5, f"oracle parsing feats {i}")
+        assert_close(ours[i][:, :4096], gold[f"parsing_shipped/feats{i}"], 2e-5, f"product parsing feats {i}")
 
 
 def test_loss_oracle_calc_loss_matches_reference(gold):
     """calc_loss at the reference's own scales (1024 / 512 / 256): value, terms and the gradient the generator receives."""
     st = LO.loss_states(SALT)
     img, recon, _ = LO.golden_inputs()
-    r = recon[:1].clone().requires_grad_(True)
-    loss, terms = LO.calc_loss(st, img[:1], r)
-    loss.backward()
+    with torch.no_grad():
+        loss, terms = LO.calc_loss(st, img[:1], recon[:1])
     _close(loss, gold["calc_loss/loss"])
     for k in ("loss_id", "loss_l2", "loss_lpips", "loss_face_parsing"):
         _close(terms[k], gold[f"calc_loss/{k}"])
-    assert_close(r.grad[:, :, ::4, ::4], gold["calc_loss/grad_recon"], 2e-5, "d calc_loss / d recon")
+    # the fp32 gradient (1 - cosine of nearly parallel features) moves with the host CPU's thread count and vector ISA: the
+    # one in loss_vectors.npz is 5.7e-4 (max-norm) from the float64 gradient, another host's lands 1.5e-4 from it.  So it is
+    # compared in float64 with the reference's float64 gradient (oracle/make_golden_calc_loss_f64.py prints these distances)
+    g64 = np.load(os.path.join(ROOT, "tests", "golden", "calc_loss_f64.npz"))
+    st64 = {n: {k: v.double() if v.is_floating_point() else v for k, v in d.items()} for n, d in st.items()}
+    r64 = recon[:1].double().requires_grad_(True)
+    loss64, terms64 = LO.calc_loss(st64, img[:1].double(), r64)
+    loss64.backward()
+    _close(loss64, g64["loss"], 1e-9)
+    for k in ("loss_id", "loss_l2", "loss_lpips", "loss_face_parsing"):
+        _close(terms64[k], g64[k], 1e-9)
+    assert_close(r64.grad[:, :, ::4, ::4], g64["grad_recon"], 1e-6, "d calc_loss / d recon (float64)")
 
 
 def test_product_loss_modules_state_dict_contract():

@@ -903,3 +903,35 @@ def test_discriminator_matches_reference_vectors(size, batch):
     rel_l2, cos = float((a - b).norm() / b.norm()), float(torch.dot(a, b) / (a.norm() * b.norm()))
     print(f"discriminator {size} input gradient: rel-L2 {rel_l2:.2e}, cosine {cos:.6f}")
     assert rel_l2 <= 2e-2 and cos >= 0.9998, (rel_l2, cos)
+
+
+def test_bench_dump_outputs_do_not_depend_on_the_warmup(tmp_path):
+    """`bench.py --dump-outputs` writes the images of the last timed step; the noise of the timed steps is seeded after the
+    warm-up, so runs with different warm-up counts dump the same images up to the default kernels' accumulation order
+    (different noise would differ by O(1)), and they are the images an eager recomputation of those steps returns."""
+    import os
+    import subprocess
+    import sys
+    from conftest import ROOT
+    dumps = []
+    for warmup in (1, 2):
+        d = tmp_path / f"warmup{warmup}"
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--size", "256", "--batch", "2", "--steps", "2",
+                              "--warmup", str(warmup), "--no-cpu-baseline", "--no-gpu-baseline", "--no-e2e", "--faceswap-pairs", "0",
+                              "--gpen-batch", "0", "--inversion-batch", "0", "--inversion-steps", "0", "--dump-outputs", str(d)],
+                             capture_output=True, text=True, timeout=900)
+        assert out.returncode == 0, out.stderr[-2000:]
+        dumps.append(np.load(d / "image.npy"))
+    assert dumps[0].dtype == np.float32 and dumps[0].shape == (2, 3, 256, 256) and np.isfinite(dumps[0]).all()
+    assert_close(torch.from_numpy(dumps[1]), torch.from_numpy(dumps[0]), REL_TOL, "image dumped after 1 vs 2 warm-up steps")
+    # the two timed steps again, eagerly, from bench.py's rank-0 seeds: weights (build_net), codes 100, label maps 200, noise 700
+    import bench
+    from e4s_b200.masks import labelMap2OneHot
+    net = bench.build_net(256, 12, torch.device(DEV))
+    codes = cu(torch.randn(2, 12, 18, 512, generator=torch.Generator().manual_seed(100)))
+    onehot = labelMap2OneHot(cu(bench.face_label_maps(2, 12, "faces", seed=200)), 12)
+    with torch.random.fork_rng(devices=[0]), torch.no_grad():
+        torch.cuda.manual_seed(700)
+        for _ in range(2):
+            img = net.gen_img(None, codes, onehot)[0]
+    assert_close(torch.from_numpy(dumps[0]), img, REL_TOL, "dumped image vs the eager recomputation of the last timed step")
